@@ -26,13 +26,18 @@ result and the oracle; `c5` = a BASELINE configs[4]-shaped shard (12.2M rows per
 batch 8192; the true 100M-row config at N = 8), oracle-checked on the probed partitions.
 `--impl reference` times the CPU oracle alone (the reference's Rust path cannot be built
 here: no cargo, lance un-vendored), rank 0 only.
+`--dump-outputs DIR` writes what the timed search returned in its last timed step (rank 0) as
+DIR/ids.npy, DIR/distances.npy and DIR/counts.npy.  The index, the queries and hence these arrays are the
+same on every run with the same arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
 import math
 import os
+import stat
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -40,6 +45,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# cuBLAS is only run-to-run deterministic with a fixed workspace configuration; the index training below runs with
+# torch's deterministic algorithms, which require it.  Read when torch creates its first cuBLAS handle.
+os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")
 
 WORKLOADS = {
     # BASELINE.json configs[1]
@@ -147,9 +155,21 @@ def synth_vectors(cfg, n, seed, device):
 
 
 def index_cache_path(cfg, tag, device):
+    """Trained indexes are cached in a temporary directory of this user's own.  On a shared host that name can
+    already be taken by someone else: unless the directory is ours and private, returns None (train, do not cache)."""
     key = "_".join(f"{k}{cfg[k]}" for k in ("n", "dim", "nlist", "m", "metric", "data"))
     dev = "cuda" if str(device).startswith("cuda") else "cpu"
-    return f"/tmp/lancedb_b200_bench_v3_{tag}_{key}_{dev}_it{TRAIN['max_iterations']}_sr{TRAIN['sample_rate']}.npz"
+    d = os.path.join(tempfile.gettempdir(), f"lancedb_b200_bench_{os.getuid()}")
+    try:
+        os.mkdir(d, 0o700)
+        os.chmod(d, 0o700)                      # whatever the umask
+    except FileExistsError:
+        pass
+    st = os.lstat(d)
+    if not stat.S_ISDIR(st.st_mode) or st.st_uid != os.getuid() or stat.S_IMODE(st.st_mode) != 0o700:
+        log(f"[bench] {d} is not a private directory of this user: the index is not cached")
+        return None
+    return os.path.join(d, f"v3_{tag}_{key}_{dev}_it{TRAIN['max_iterations']}_sr{TRAIN['sample_rate']}.npz")
 
 
 def get_index(cfg, tag, device):
@@ -158,7 +178,7 @@ def get_index(cfg, tag, device):
     from lancedb_b200.index import IvfPqIndexData, train_ivf_pq
     import torch
     path = index_cache_path(cfg, tag, device)
-    if os.path.exists(path):
+    if path is not None and os.path.exists(path):
         z = np.load(path)
         ix = IvfPqIndexData(int(z["dim"]), int(z["nlist"]), int(z["m"]), str(z["metric"]), z["centroids"],
                             z["codebook"], z["part_offsets"], z["codes_t"], z["row_ids"], None)
@@ -166,8 +186,16 @@ def get_index(cfg, tag, device):
     t0 = time.time()
     x = synth_vectors(cfg, cfg["n"], 42, device)
     t1 = time.time()
-    ix = train_ivf_pq(x, num_partitions=cfg["nlist"], num_sub_vectors=cfg["m"], distance_type=cfg["metric"],
-                      max_iterations=TRAIN["max_iterations"], sample_rate=TRAIN["sample_rate"], device=device)
+    # the k-means updates (index_add_ / scatter_add_) sum with float atomics on CUDA unless torch is asked for its
+    # deterministic kernels: without them every training run yields a slightly different index.  An op without a
+    # deterministic kernel raises here rather than quietly making the index vary from run to run.
+    mode = (torch.are_deterministic_algorithms_enabled(), torch.is_deterministic_algorithms_warn_only_enabled())
+    torch.use_deterministic_algorithms(True)
+    try:
+        ix = train_ivf_pq(x, num_partitions=cfg["nlist"], num_sub_vectors=cfg["m"], distance_type=cfg["metric"],
+                          max_iterations=TRAIN["max_iterations"], sample_rate=TRAIN["sample_rate"], device=device)
+    finally:
+        torch.use_deterministic_algorithms(mode[0], warn_only=mode[1])
     build_s = time.time() - t1
     gq = synth_vectors(cfg, 128, 4343, device)
     xs = x / x.norm(dim=1, keepdim=True) if cfg["metric"] == "cosine" else x
@@ -176,12 +204,13 @@ def get_index(cfg, tag, device):
     gt = d.topk(cfg["k"], largest=False).indices.cpu().numpy().astype(np.uint64)
     gqn = gq.cpu().numpy()
     del x, xs, d
-    tmp = path + f".{os.getpid()}.tmp.npz"
-    np.savez(tmp, dim=ix.dim, nlist=ix.nlist, m=ix.m, metric=ix.metric, centroids=ix.centroids,
-             codebook=ix.codebook, part_offsets=ix.part_offsets, codes_t=ix.codes_t, row_ids=ix.row_ids,
-             gt_queries=gqn, gt_ids=gt, build_s=build_s)
-    os.replace(tmp, path)
-    log(f"[bench] index built in {time.time() - t0:.1f}s (training+encoding {build_s:.1f}s) -> {path}")
+    if path is not None:
+        tmp = path + f".{os.getpid()}.tmp.npz"
+        np.savez(tmp, dim=ix.dim, nlist=ix.nlist, m=ix.m, metric=ix.metric, centroids=ix.centroids,
+                 codebook=ix.codebook, part_offsets=ix.part_offsets, codes_t=ix.codes_t, row_ids=ix.row_ids,
+                 gt_queries=gqn, gt_ids=gt, build_s=build_s)
+        os.replace(tmp, path)
+    log(f"[bench] index built in {time.time() - t0:.1f}s (training+encoding {build_s:.1f}s) -> {path or 'not cached'}")
     return ix, gqn, gt, build_s
 
 
@@ -352,8 +381,10 @@ def run_reference(args, cfg):
         orc.search(q[i % nb][: max(threads, B // 8)], k=cfg["k"], nprobes=cfg["nprobes"], nthreads=threads)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        orc.search(q[i % nb], k=cfg["k"], nprobes=cfg["nprobes"], nthreads=threads)
+        res = orc.search(q[i % nb], k=cfg["k"], nprobes=cfg["nprobes"], nthreads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res)
     qps = B * args.steps / dt
     gi, _, _ = orc.search(gq, k=cfg["k"], nprobes=cfg["nprobes"], nthreads=threads)
     recall = float(np.mean([len(set(gi[i].tolist()) & set(gt[i].tolist())) / cfg["k"] for i in range(len(gq))]))
@@ -409,6 +440,17 @@ def recall_of(ids, gt, k):
 def same(a, b):
     return bool(np.array_equal(a[0], b[0]) and np.array_equal(np.asarray(a[1]).view(np.uint32), np.asarray(b[1]).view(np.uint32))
                 and np.array_equal(np.asarray(a[2]).view(np.uint32), np.asarray(b[2]).view(np.uint32)))
+
+
+def dump_outputs(out_dir, ids, dist, cnt):
+    """One search's results as a caller receives them: ids [B,k] u64, distances [B,k] f32, counts [B] u32.  Ids and
+    counts are stored as float64 (exact below 2**53; an empty slot's id UINT64_MAX reads 2**64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"ids": np.asarray(ids).view(np.uint64).astype(np.float64),
+              "distances": np.asarray(dist, np.float32),
+              "counts": np.asarray(cnt).view(np.uint32).astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------ timing helpers
@@ -568,7 +610,11 @@ def main():
     ap.add_argument("--parallelism", default="replicas", choices=["replicas", "sharded"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip latency / extra_workloads / sharded / c5 blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's ids / distances / counts as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = WORKLOADS[args.workload]
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     if args.impl == "reference":
@@ -677,6 +723,8 @@ def main():
         ev[i][1].record()
     barrier()
     launches = _native.kernel_launch_count() - launches0
+    if args.dump_outputs and rank == 0:            # before the regions below overwrite d_ids / d_dist / d_cnt
+        dump_outputs(args.dump_outputs, d_ids.cpu().numpy(), d_dist.cpu().numpy(), d_cnt.cpu().numpy())
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=device)
     if world > 1:

@@ -381,3 +381,38 @@ def test_index_loaded_from_lance_files_searches_like_the_in_memory_one(tmp_path)
         assert a["_rowid"].to_pylist() == b["_rowid"].to_pylist()
         assert np.array_equal(np.asarray(a["_distance"].to_pylist(), np.float32).view(np.uint32),
                               np.asarray(b["_distance"].to_pylist(), np.float32).view(np.uint32))
+
+
+_BENCH_LAST_STEP_SCRIPT = r"""
+import sys, numpy as np
+sys.path.insert(0, {root!r})
+import bench, oracle
+cfg = bench.WORKLOADS["tiny"]
+ix = bench.get_index(cfg, "tiny", "cuda:0")[0]          # the index the run trained (read back from its cache)
+q = bench.synth_vectors(cfg, 8 * cfg["batch"], 43, "cuda:0").reshape(8, cfg["batch"], cfg["dim"])[{step} % 8]
+ids, dist, cnt = oracle.OracleIndex.from_data(ix).search(q.cpu().numpy(), k=cfg["k"], nprobes=cfg["nprobes"])
+np.savez({dst!r}, ids=ids, distances=dist, counts=cnt)
+"""
+
+
+def test_bench_dump_outputs_reproducible_and_equal_to_the_oracle(tmp_path):
+    """bench.py --dump-outputs on the timed device-resident path: two runs that each train their index on the GPU dump
+    the same bytes, and the dump is the oracle's answer for the last timed step's batch (queries 8 batches deep, step
+    i searches batch i % 8).  The bench inherits the suite's LGPU_SMALL_SLOTS=0, so its tiny batches take the batched
+    kernels that the flagship workload times."""
+    import os, subprocess, sys
+    from tests.util import bench_dumps
+    steps = 5
+    (a, da), (b, _) = bench_dumps(tmp_path, "--workload", "tiny", "--steps", str(steps), "--warmup", "3",
+                                  "--no-cpu-baseline")
+    assert da["steps"] == steps and da["gate"]["gpu_equals_oracle_plain"]
+    for name in ("ids", "distances", "counts"):
+        assert np.array_equal(a[name], b[name]), name
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dst = str(tmp_path / "want.npz")
+    subprocess.run([sys.executable, "-c", _BENCH_LAST_STEP_SCRIPT.format(root=root, step=steps - 1, dst=dst)],
+                   check=True, timeout=300, cwd=root, env=dict(os.environ, TMPDIR=str(tmp_path / "tmp0")))
+    want = np.load(dst)
+    assert np.array_equal(a["ids"], want["ids"].astype(np.float64))
+    assert np.array_equal(a["distances"].view(np.uint32), want["distances"].view(np.uint32))
+    assert np.array_equal(a["counts"], want["counts"].astype(np.float64))

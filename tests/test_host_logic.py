@@ -248,6 +248,39 @@ def test_bench_reference_arm_prints_one_json_line(tmp_path):
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and "workload" in d["config"]
 
 
+def test_bench_dump_outputs_reproducible(tmp_path):
+    """bench.py --dump-outputs writes the last timed step's results (ids / distances / counts of the whole batch), and
+    two runs that each train their own index write the same bytes."""
+    from tests.util import bench_dumps
+    (a, da), (b, _) = bench_dumps(tmp_path, "--impl", "reference", "--workload", "tiny", "--steps", "2", "--warmup", "1")
+    assert da["steps"] == 2
+    assert sorted(a) == ["counts", "distances", "ids"]
+    assert a["ids"].shape == a["distances"].shape == (64, 10) and a["counts"].shape == (64,)
+    assert a["ids"].dtype == a["counts"].dtype == np.float64 and a["distances"].dtype == np.float32
+    assert np.all(a["counts"] == 10) and np.all(np.diff(a["distances"], axis=1) >= 0)
+    for name in a:
+        assert np.array_equal(a[name], b[name]), name
+
+
+def test_bench_index_cache_only_in_a_private_directory_of_this_user(tmp_path, monkeypatch):
+    """bench.py caches trained indexes in <tmp>/lancedb_b200_bench_<uid>, created 0700; a directory of that name that
+    is not this user's private directory (other mode, a link) is not used and nothing is cached."""
+    import importlib, stat, tempfile
+    monkeypatch.setenv("CUBLAS_WORKSPACE_CONFIG", os.environ.get("CUBLAS_WORKSPACE_CONFIG", ":4096:8"))
+    bench = importlib.import_module("bench")
+    monkeypatch.setattr(tempfile, "tempdir", str(tmp_path))
+    cfg = bench.WORKLOADS["tiny"]
+    d = str(tmp_path / f"lancedb_b200_bench_{os.getuid()}")
+    path = bench.index_cache_path(cfg, "tiny", "cpu")
+    assert os.path.dirname(path) == d and stat.S_IMODE(os.lstat(d).st_mode) == 0o700
+    assert bench.index_cache_path(cfg, "tiny", "cpu") == path
+    os.chmod(d, 0o755)
+    assert bench.index_cache_path(cfg, "tiny", "cpu") is None
+    os.rmdir(d)
+    os.symlink(str(tmp_path), d)
+    assert bench.index_cache_path(cfg, "tiny", "cpu") is None
+
+
 def test_oracle_pq_encode_is_argmin_of_the_distance_table():
     """orc_pq_encode picks, per sub-vector, the first minimum of the very table row orc_build_lut produces for
     the row's residual; orc_ivf_assign is find_partitions with nprobes 1."""

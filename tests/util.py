@@ -64,6 +64,22 @@ def load_golden(metric):
     return ix, g("queries"), cases, flat
 
 
+def bench_dumps(tmp_path, *args, runs=2):
+    """Runs `bench.py --dump-outputs` `runs` times, each with a temporary directory of its own (so every run trains
+    its index afresh) and returns the dumped arrays of each run as {name: array} plus its JSON line."""
+    import json, os, subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = []
+    for r in range(runs):
+        tmp, dump = tmp_path / f"tmp{r}", tmp_path / f"dump{r}"
+        tmp.mkdir()
+        proc = subprocess.run([sys.executable, os.path.join(root, "bench.py"), *args, "--dump-outputs", str(dump)],
+                              capture_output=True, text=True, timeout=900, cwd=root, env=dict(os.environ, TMPDIR=str(tmp)))
+        assert proc.returncode == 0, proc.stderr[-2000:]
+        out.append(({f[:-4]: np.load(dump / f) for f in sorted(os.listdir(dump))}, json.loads(proc.stdout)))
+    return out
+
+
 def same_result(got, want):
     gi, gd, gc = got
     wi, wd, wc = want
